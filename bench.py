@@ -42,6 +42,7 @@ MULS_PER_NTT = (N // 2) * LOG_N          # 201 326 592 (SURVEY §8d)
 ALG_BYTES_PER_NTT = 16 * N               # one read + one write of the data (SURVEY §8d)
 METRIC = "field-muls/s on 2^24-coeff 64-bit-prime NTT"
 UNIT = "field-muls/s"
+DUMP_SAMPLE = 1 << 20                    # output coefficients --dump-outputs writes, over all ranks
 
 
 def measured_peaks():
@@ -175,6 +176,21 @@ def horner_spots(a_host, X_host, log_n, ks):
     return all(int(X_host[k]) == oracle.poly_eval_horner(GL, a_host, pow(w, k, GL)) for k in ks)
 
 
+def dump_outputs(out_dir, x, rank, world):
+    """--dump-outputs: what the last timed step left in the 2^24-coefficient operand (u64 mod p), as a fixed sample
+    of DUMP_SAMPLE coefficients over all ranks (seed 0, sorted): the indices and values as float64 (values rounded
+    to 53 bits) and the values exactly as four 16-bit limbs, least significant first, in float32."""
+    import numpy as np
+    idx = np.sort(np.random.default_rng(0).choice(N, DUMP_SAMPLE // world, replace=False))
+    v = x[idx]
+    limbs = np.stack([(v >> np.uint64(16 * k)) & np.uint64(0xFFFF) for k in range(4)], axis=1)
+    suffix = "" if world == 1 else f"_rank{rank}"
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"ntt_out_index{suffix}.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, f"ntt_out{suffix}.npy"), v.astype(np.float64))
+    np.save(os.path.join(out_dir, f"ntt_out_u16{suffix}.npy"), limbs.astype(np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -184,7 +200,11 @@ def main():
     ap.add_argument("--ref-threads", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the `configs` / `multi` blocks (A/B timing runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a seeded sample of the last timed step's output to DIR/*.npy (32 MiB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 
     if args.impl == "reference":
@@ -263,6 +283,7 @@ def main():
     launches = ctx.launches - launches0
     ms_per_step = max_over_ranks(e0.elapsed_time(e1)) / args.steps
     value = world * MULS_PER_NTT / (ms_per_step * 1e-3)
+    last_output = ops.to_host(data) if args.dump_outputs else None   # region 2 transforms `data` again
 
     # ---- timed region 2: per-kernel durations (CUDA events around every launch, same stream) ----
     ctx.prof_enable(True)
@@ -316,7 +337,6 @@ def main():
     hosts = [torch.empty(N, dtype=torch.int64).pin_memory() for _ in range(SLOTS)]
     for h in hosts:
         h.copy_(data.cpu())
-    e2e_steps = max(4, min(args.steps, 12))
 
     def e2e_run(steps):
         for i in range(steps):
@@ -329,9 +349,9 @@ def main():
     e2e_run(4)
     barrier()
     t0 = time.perf_counter()
-    e2e_run(e2e_steps)
+    e2e_run(args.steps)
     torch.cuda.synchronize()
-    e2e_mine = (time.perf_counter() - t0) / e2e_steps
+    e2e_mine = (time.perf_counter() - t0) / args.steps
     e2e_s = max_over_ranks(e2e_mine)
     e2e_value = world * MULS_PER_NTT / e2e_s
     copy_gbs = 2 * 8 * N / e2e_mine / 1e9   # this rank's H2D + D2H bytes per second while all N ranks copy
@@ -376,6 +396,10 @@ def main():
         cpu_baseline = {"value": MULS_PER_NTT / secs, "unit": UNIT, "cores": 1, "kind": "port",
                         "sample": "one full 2^24-point faithful recursive fft (polynomial/mod.rs:295-323 restated in C), "
                                   f"single thread as in the reference, {secs:.2f} s; host has {os.cpu_count()} cores"}
+
+    if last_output is not None:
+        dump_outputs(args.dump_outputs, last_output, rank, world)
+        del last_output
 
     if rank == 0:
         line = {

@@ -1,5 +1,5 @@
-import numpy as np, torch, sys
-sys.path.insert(0,'/root/repo')
+import numpy as np, torch, os, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import oracle
 from ronkathon_b200 import Context, ops
 torch.cuda.set_device(0)
